@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- molecules/sec of the SphereNet QM9-shape hot path (BASELINE.json metric, configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--quick]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--quick] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (SphereNet 4-layer h=128 forward: radius graph -> geometry ->
 basis -> 4 interaction blocks -> readout) over one synthetic batch of 128 QM9-shaped molecules per
@@ -12,13 +12,20 @@ GPU (weak scaling: per-GPU work fixed).  Prints ONE JSON line (rank 0).
              repeated (`windows`), `value` is the MEDIAN window and min / max are reported beside it.
   e2e        same metric through the public class API (model(batch)) with HOST (pinned) inputs:
              H2D of z/pos/batch and D2H of the energies inside the timed region, every step
-  roofline   the dominant kernel, timed with CUDA events in a separate pass (per entry point of the C ABI)
+  roofline   the dominant kernel, timed with CUDA events in a separate pass (per entry point of the C ABI) over
+             min(K, 10) steps (`roofline.steps`): per-kernel means, not a throughput
   parity     the energies of the timed batches vs the oracle's op sequence on the same GPU (rel err, asserted < 1e-5)
   cpu_baseline  the travelling oracle (oracle/restated.py == the reference's algorithm, bit-identical
              to the real reference on CPU) on this box's host cores, bounded sample
-  train      BASELINE configs[4]: forward + backward + overlapped gradient all-reduce + fused Adam step
-  --impl reference   times that same CPU implementation as the reference arm on the SAME 128-molecule batches
+  train      BASELINE configs[4]: forward + backward + overlapped gradient all-reduce + fused Adam step; windows of
+             min(max(K, 3), 30) steps (`train.steps`), so that a long headline run does not spend minutes on this
+             secondary number
+  --impl reference   times that same CPU implementation as the reference arm on the SAME 128-molecule batches, exactly
+             K steps after W (at least 1) warm-up steps, ~1.5 s per step
              (the real reference is Python over uninstallable PyG wheels; its restatement is what travels)
+  --dump-outputs DIR  after the timed steps, the energies the timed loop returned for its last step (rank 0's
+             batch (K - 1) mod 8, float32 [128, 1]) as DIR/energy.npy, in either arm: the inputs and weights are seeded,
+             so two builds, or a build and the reference arm, run with the same arguments can be compared output for output
 """
 import argparse
 import json
@@ -30,6 +37,8 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # no bytecode caches in the tree it runs from, which may be read-only (build() has
+                                 # already run there, so the build() call below finds the library up to date)
 
 MOLS_PER_GPU = 128
 N_ROTATE = 8                     # distinct batches cycled through the timed region
@@ -186,16 +195,19 @@ def run_reference_arm(args):
     sd = {k: v.detach() for k, v in bench_model(torch).state_dict().items()}
     cores = pick_cpu_threads(sd, restated, torch)
     batches = bench_batches(0)
-    steps = max(1, min(args.steps, 60))            # ~1.5 s per 128-molecule step: a few minutes at most
+    steps = args.steps
+    args.warmup = max(args.warmup, 1)
     with torch.no_grad():
-        for s in range(max(1, min(args.warmup, 2))):
+        for s in range(args.warmup):
             b = batches[s % N_ROTATE]
             restated.spherenet_forward(sd, b.z, b.pos, b.batch)
         t0 = time.perf_counter()
         for s in range(steps):
             b = batches[s % N_ROTATE]
-            restated.spherenet_forward(sd, b.z, b.pos, b.batch)
+            energy = restated.spherenet_forward(sd, b.z, b.pos, b.batch)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, energy)
     val = MOLS_PER_GPU * steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "molecules/s",
             "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / steps,
@@ -208,6 +220,13 @@ def run_reference_arm(args):
             "e2e": {"value": val, "unit": "molecules/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir, energy):
+    """--dump-outputs: the energies of the last timed step as out_dir/energy.npy, float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "energy.npy"), energy.detach().cpu().numpy().astype(np.float32))
 
 
 def time_ms(torch, fn, n=10, warm=3):
@@ -350,7 +369,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline + roofline only (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the energies of the last timed step as DIR/energy.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -441,6 +464,7 @@ def main():
     pipe_r = InferencePipeline(model, dev, depth=depth)
     pending, pending_r = [], []
     checksum = [0.0]
+    last_r = [None]                                       # host energies of the latest step step_resident_pipelined took
 
     def step_e2e_pipelined(s):
         pending.append(pipe.submit(host[s % N_ROTATE]))
@@ -454,7 +478,7 @@ def main():
         pending_r.append(pipe_r.submit(resident[s % N_ROTATE]))
         last = (s == args.steps - 1)
         while len(pending_r) > (0 if last else depth - 1):
-            pipe_r.result(pending_r.pop(0))
+            last_r[0] = pipe_r.result(pending_r.pop(0))
 
     def join_streams():
         cur = torch.cuda.current_stream()
@@ -481,6 +505,10 @@ def main():
     if depth > 1:
         dev_w, wall_w = windows(step_resident_pipelined, args.steps, join=join_streams)
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        # what the loop behind `value` returned for its last timed step (pipe_r takes no further batches, so its host
+        # buffer still holds them)
+        dump_outputs(args.dump_outputs, last_r[0] if depth > 1 else sink[-1])
     ms = statistics.median(dev_w)
     ms_serial = statistics.median(dev_serial_w)
     wall_e2e_serial = statistics.median(e2e_wall_w)
@@ -578,7 +606,7 @@ def main():
             traffic = json.load(fh).get(dom.replace("dig3d_", ""))
     ach = (flops_d / (dom_ms * 1e-3) / 1e12) if bound == "tensor" else (bytes_d / (dom_ms * 1e-3) / 1e9)
     peak = tf_peak if bound == "tensor" else hbm_peak
-    roof = {"kernel": dom.replace("dig3d_", ""), "bound": bound, "achieved": ach, "peak": peak,
+    roof = {"kernel": dom.replace("dig3d_", ""), "steps": n_roof, "bound": bound, "achieved": ach, "peak": peak,
             "unit": "TFLOP/s" if bound == "tensor" else "GB/s", "frac": ach / peak if peak else None,
             "traffic": traffic, "traffic_source": "profiles/r02_dram_traffic.json (ncu --set full, dram__bytes_read.sum + dram__bytes_write.sum per launch)" if traffic else None,
             "peak_source": f"{which} " + ("bf16_tflops_sustained (kernel timed inside the step; kind::f16 MMAs run at the bf16 rate)" if bound == "tensor" else "hbm_gbs"),

@@ -18,6 +18,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from oracle import FIXTURE_THREADS  # noqa: E402
 from oracle.ref_loader import load_reference, load_reference_utils  # noqa: E402
 from oracle.weights import formula_state_dict  # noqa: E402
 from dig_b200.data import synthetic_batch, Batch  # noqa: E402
@@ -167,6 +168,7 @@ def state_shapes(method):
 
 
 def main():
+    torch.set_num_threads(FIXTURE_THREADS)
     os.makedirs(GOLD, exist_ok=True)
     method = load_reference()
     utils = load_reference_utils()

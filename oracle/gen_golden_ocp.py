@@ -13,6 +13,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from oracle import FIXTURE_THREADS  # noqa: E402
 from oracle.ocp_stub import OCP_DIR, load_comenet_ocp  # noqa: E402
 from oracle.weights import formula_state_dict  # noqa: E402
 from dig_b200.data import synthetic_pbc_batch  # noqa: E402
@@ -25,6 +26,7 @@ WSEED = 21
 
 
 def main():
+    torch.set_num_threads(FIXTURE_THREADS)
     mod = load_comenet_ocp()
     torch.manual_seed(0)
     model = mod.ComENet(**CTOR)

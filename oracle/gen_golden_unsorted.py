@@ -14,11 +14,12 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 from oracle.ref_loader import load_reference_utils  # noqa: E402
-from oracle import shim  # noqa: E402
+from oracle import FIXTURE_THREADS, shim  # noqa: E402
 from dig_b200.data import synthetic_batch  # noqa: E402
 
 
 def main():
+    torch.set_num_threads(FIXTURE_THREADS)
     utils = load_reference_utils()
     b = synthetic_batch(3, "qm9", seed=9, variable=True)
     ei = shim.radius_graph(b.pos, 5.0, b.batch)

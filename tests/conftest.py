@@ -10,19 +10,14 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
     has_gpu = torch.cuda.is_available()
-    from oracle.ref_loader import reference_available
-    has_ref = reference_available()
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
 
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
